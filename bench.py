@@ -11,6 +11,8 @@ Batch-sharded over N GPUs with no data-path collective (weak scaling).
           H2D every timestep and the stage-4 feature map read back D2H every timestep
   --impl reference : the reference's CPU path (oracle port, torch fp32, all host threads) on a
           bounded sample of the same workload.
+  --dump-outputs DIR : also write what the last timed step computed (dump_outputs); the inputs and
+          weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -438,6 +440,25 @@ def run_train(args, rank, world, local_rank):
         dist.destroy_process_group()
 
 
+DUMP_MAX_ELEMS = 1 << 21      # per array (8 MB of float32): the eight state arrays of RVT-B stay below 64 MB in all
+
+
+def dump_outputs(out_dir, states):
+    """Write what one timed step returns -- the final (h, c) of every stage, NCHW float32 -- as
+    out_dir/stage<s>_h.npy and out_dir/stage<s>_c.npy (s = 1..4).  An array of more than DUMP_MAX_ELEMS
+    elements is written as a fixed sample: the values at DUMP_MAX_ELEMS ascending flat NCHW positions
+    drawn with seed 0, the same positions on every run, so two builds can be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for s, (h, c) in enumerate(states, 1):
+        for name, t in (('h', h), ('c', c)):
+            a = t.float().contiguous().cpu().numpy()
+            if a.size > DUMP_MAX_ELEMS:
+                idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+                a = a.reshape(-1)[idx]
+            np.save(os.path.join(out_dir, f'stage{s}_{name}.npy'), a)
+
+
 def count_kernel_launches(fn, dev):
     """MEASURED number of GPU kernels one call of `fn` launches (CUPTI activity records through torch.profiler; kernels
     launched by CUDA-graph replay and through the ctypes C-ABI are included).  Returns (count, {name: count})."""
@@ -601,7 +622,13 @@ def main():
     ap.add_argument('--no-wavefront', action='store_true', help='run the four stages strictly one after the other')
     ap.add_argument('--extras', default='train,voxel,eager_gpu,dropin,rvt_s_gen1_bs64',
                     help='comma list of the extra legs reported under "extra" (empty string: none)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the final states of the last timed step (rank 0) to DIR/*.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.mode != 'infer'):
+        ap.error('--dump-outputs applies to the inference benchmark (--impl ours --mode infer)')
 
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -687,16 +714,17 @@ def main():
         torch.cuda.synchronize(dev)
 
     def timed(fn, steps):
+        """(device ms of `steps` calls of fn, what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize(dev)
         ms = sharding.max_over_ranks(e0.elapsed_time(e1), dev)     # device time, max over ranks
         barrier()
-        return ms
+        return ms, out
 
     with torch.inference_mode():
         if args.no_graph:
@@ -710,11 +738,13 @@ def main():
         sampler = ClockSampler(local_rank)
         if rank == 0:
             sampler.start()
-        ms = timed(step_resident, args.steps)
+        ms, last_states = timed(step_resident, args.steps)
         clocks = sampler.stop() if rank == 0 else None
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, last_states)
         for _ in range(3):
             step_e2e()
-        ms_e2e = timed(step_e2e, args.steps)
+        ms_e2e, _ = timed(step_e2e, args.steps)
         launches_per_step, launch_names = (None, {})
         if rank == 0:
             launches_per_step, launch_names = count_kernel_launches(step_resident, dev)

@@ -26,7 +26,7 @@ from tests.golden_configs import (BACKBONE_CASES, MIXED_DENSITY_CASES, VOXEL_CAS
                                   spec_of)
 from oracle import neighbours_oracle as no  # noqa: E402
 from oracle import detection_oracle as do  # noqa: E402
-from tests.golden_configs import DETECTION_CASES, POSTPROCESS_CASES, detection_inputs  # noqa: E402
+from tests.golden_configs import DETECTION_CASES, DETECTOR_CASES, POSTPROCESS_CASES, detection_inputs  # noqa: E402
 from tests.helpers import GRAD_CASES, grad_sub, case_inputs, train_loss  # noqa: E402
 
 from models.detection.recurrent_backbone import build_recurrent_backbone  # noqa: E402
@@ -215,6 +215,51 @@ def run_detection_cases():
     np.savez_compressed(os.path.join(GOLD, 'det.npz'), **out)
 
 
+def state_layout(sd):
+    """{key: [shape, dtype name]} of a state_dict"""
+    return {k: [list(v.shape), str(v.dtype).replace('torch.', '')] for k, v in sd.items()}
+
+
+def run_reference_detector_cases():
+    """INTEGRATION.md section 1: the reference's own YoloXDetector built around rvt_b200's backbone (its PAFPN / YOLOX head
+    sized from our get_stage_dims / get_strides) has the reference detector's state_dict, and checkpoints load strictly both
+    ways.  The model config, the reference detector's state_dict layout, stage dims and strides go to
+    tests/golden/reference_detector.json (tests/test_reference_integration_cpu.py)."""
+    import json
+    import yaml
+    import models.detection.yolox_extension.models.detector as det
+    import rvt_b200
+    out = {}
+    for embed_dim, dim_head in DETECTOR_CASES:
+        with open(os.path.join(_refshim.REFERENCE_ROOT, 'config', 'model', 'maxvit_yolox', 'default.yaml')) as f:
+            cfg = yaml.safe_load(f)['model']
+        cfg['backbone']['embed_dim'] = embed_dim
+        cfg['backbone']['stage']['attention']['dim_head'] = dim_head
+        cfg['backbone']['stage']['attention']['partition_size'] = [6, 10]    # what config/modifier.py:36-41 derives for 1Mpx
+        cfg['backbone']['stage']['attention']['ls_init_value'] = 1e-5        # (PyYAML reads the literal 1e-5 as a string)
+        cfg['backbone']['in_res_hw'] = [384, 640]
+        cfg['head']['num_classes'] = 3
+        ref_model = det.YoloXDetector(_refshim.DictConfig(cfg))
+        ref_builder = det.build_recurrent_backbone
+        det.build_recurrent_backbone = rvt_b200.build_recurrent_backbone
+        try:
+            our_model = det.YoloXDetector(_refshim.DictConfig(cfg))             # reference FPN + head around rvt_b200.RNNDetector
+        finally:
+            det.build_recurrent_backbone = ref_builder
+        assert isinstance(our_model.backbone, rvt_b200.RNNDetector)
+        layout = state_layout(ref_model.state_dict())
+        assert state_layout(our_model.state_dict()) == layout
+        our_model.load_state_dict(ref_model.state_dict(), strict=True)
+        ref_model.load_state_dict(our_model.state_dict(), strict=True)
+        dims, strides = ref_model.backbone.get_stage_dims((2, 3, 4)), ref_model.backbone.get_strides((2, 3, 4))
+        assert our_model.backbone.get_stage_dims((2, 3, 4)) == dims and our_model.backbone.get_strides((2, 3, 4)) == strides
+        out[f'{embed_dim}_{dim_head}'] = dict(model_cfg=cfg, state_dict=layout, stage_dims=list(dims), strides=list(strides))
+        print(f'detector {embed_dim}/{dim_head}: reference detector around rvt_b200 backbone matches, {len(layout)} entries')
+    with open(os.path.join(GOLD, 'reference_detector.json'), 'w') as f:
+        json.dump(out, f, sort_keys=True)
+        f.write('\n')
+
+
 def run_neighbour_cases():
     """SURVEY 8 f4: oracle.neighbours_oracle vs the reference's own code; the REFERENCE's outputs go to tests/golden/neigh.npz"""
     out = {}
@@ -268,6 +313,8 @@ if __name__ == '__main__':
         run_neighbour_cases()
     if '--grads-only' not in sys.argv and want('det'):
         run_detection_cases()
+    if '--grads-only' not in sys.argv and want('reference_detector'):
+        run_reference_detector_cases()
     if '--grads-only' not in sys.argv:
         for n, c in VOXEL_CASES.items():
             if want(n):

@@ -108,6 +108,8 @@ POSTPROCESS_CASES = {
     'pp_gen4': dict(seed=5, batch=3, anchors=5040, num_classes=3, conf=0.1, nms=0.45),
     'pp_small': dict(seed=6, batch=2, anchors=300, num_classes=2, conf=0.3, nms=0.45),
 }
+# whole detector (backbone + PAFPN + YOLOX head) at 1Mpx: (embed_dim, dim_head) of RVT-B / S / T
+DETECTOR_CASES = [(64, 32), (48, 24), (32, 32)]
 
 
 def detection_inputs(case):

@@ -1,53 +1,58 @@
-"""CPU, build container only (skipped where /root/reference is absent, e.g. on the GPU box): the drop-in claim of
-INTEGRATION.md §1 exercised against the REAL reference — the reference's own ``YoloXDetector`` is constructed with
-``build_recurrent_backbone`` pointed at ``rvt_b200``; its PAFPN / YOLOX head are sized from our ``get_stage_dims`` /
-``get_strides``; the reference backbone's checkpoint keys load strictly into ours and vice versa."""
+"""CPU: the drop-in claim of INTEGRATION.md §1 against the REAL reference's detector, as recorded in
+tests/golden/reference_detector.json by oracle/make_golden.py.  There the reference's own ``YoloXDetector`` was built around
+``rvt_b200``'s backbone (``build_recurrent_backbone`` pointed at ``rvt_b200``), checked, and its model config, state_dict
+layout (keys, shapes, dtypes), stage dims and strides recorded.  Here ``rvt_b200``'s detector, whose PAFPN / YOLOX head are
+sized from our ``get_stage_dims`` / ``get_strides``, must reproduce that layout, and a checkpoint with the reference
+detector's layout must load strictly into it and round-trip."""
+import json
 import os
-import sys
 
 import pytest
 import torch
-import yaml
 
-REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'models')), reason='reference tree not present')
+import rvt_b200
+from rvt_b200.detection import YoloXDetector
+from tests.golden_configs import DETECTOR_CASES
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_detector.json')
 
 
 @pytest.fixture(scope='module')
-def ref_modules():
-    from oracle import _refshim
-    _refshim.install()
-    import models.detection.yolox_extension.models.detector as det
-    return det, _refshim
+def reference():
+    with open(GOLDEN) as f:
+        return json.load(f)
 
 
-def _model_cfg(shim, embed_dim=64, dim_head=32):
-    cfg = yaml.safe_load(open(os.path.join(REF, 'config', 'model', 'maxvit_yolox', 'default.yaml')))['model']
-    cfg['backbone']['embed_dim'] = embed_dim
-    cfg['backbone']['stage']['attention']['dim_head'] = dim_head
-    cfg['backbone']['stage']['attention']['partition_size'] = (6, 10)       # what config/modifier.py:36-41 derives for 1Mpx
-    cfg['backbone']['stage']['attention']['ls_init_value'] = 1e-5           # (PyYAML reads the literal 1e-5 as a string)
-    cfg['backbone']['in_res_hw'] = (384, 640)
-    cfg['head']['num_classes'] = 3
-    return shim.DictConfig(cfg)
+def _layout(sd):
+    return {k: [list(v.shape), str(v.dtype).replace('torch.', '')] for k, v in sd.items()}
 
 
-@pytest.mark.parametrize('embed_dim,dim_head', [(64, 32), (48, 24), (32, 32)])       # RVT-B / S / T
-def test_reference_detector_builds_around_our_backbone(ref_modules, monkeypatch, embed_dim, dim_head):
-    det, shim = ref_modules
-    import rvt_b200
-    cfg = _model_cfg(shim, embed_dim, dim_head)
-    ref_model = det.YoloXDetector(cfg)                                       # the reference's own backbone
-    monkeypatch.setattr(det, 'build_recurrent_backbone', rvt_b200.build_recurrent_backbone)
-    our_model = det.YoloXDetector(cfg)                                       # reference FPN + head around rvt_b200.RNNDetector
-    assert isinstance(our_model.backbone, rvt_b200.RNNDetector)
-    # FPN / head were sized from our get_stage_dims / get_strides exactly as from the reference's
-    ref_sd, our_sd = ref_model.state_dict(), our_model.state_dict()
-    assert {k: tuple(v.shape) for k, v in ref_sd.items()} == {k: tuple(v.shape) for k, v in our_sd.items()}
+def _checkpoint(layout, seed):
+    """seeded state_dict with the given layout (stands in for a reference checkpoint)"""
+    g = torch.Generator().manual_seed(seed)
+    sd = {}
+    for k, (shape, dtype) in layout.items():
+        dt = getattr(torch, dtype)
+        sd[k] = (torch.randn(shape, generator=g).to(dt) if dt.is_floating_point else
+                 torch.randint(0, 1000, tuple(shape), generator=g, dtype=dt))
+    return sd
+
+
+@pytest.mark.parametrize('embed_dim,dim_head', DETECTOR_CASES)       # RVT-B / S / T
+def test_reference_detector_builds_around_our_backbone(reference, embed_dim, dim_head):
+    ref = reference[f'{embed_dim}_{dim_head}']
+    model = YoloXDetector(ref['model_cfg'])
+    assert isinstance(model.backbone, rvt_b200.RNNDetector)
+    # FPN / head were sized from our get_stage_dims / get_strides exactly as the reference sized them from its own backbone
+    assert list(model.backbone.get_stage_dims((2, 3, 4))) == ref['stage_dims']
+    assert list(model.backbone.get_strides((2, 3, 4))) == ref['strides']
+    assert _layout(model.state_dict()) == ref['state_dict']
     # a reference checkpoint loads strictly (whole detector, Lightning strips the 'mdl.' prefix) and round-trips
-    our_model.load_state_dict(ref_sd, strict=True)
-    for k, v in our_model.backbone.state_dict().items():
-        assert torch.equal(v, ref_sd['backbone.' + k]), k
-    ref_model.load_state_dict(our_model.state_dict(), strict=True)
-    assert our_model.backbone.get_stage_dims((2, 3, 4)) == ref_model.backbone.get_stage_dims((2, 3, 4))
-    assert our_model.backbone.get_strides((2, 3, 4)) == ref_model.backbone.get_strides((2, 3, 4))
+    ckpt = _checkpoint(ref['state_dict'], embed_dim * 100 + dim_head)
+    model.load_state_dict(ckpt, strict=True)
+    for k, v in model.backbone.state_dict().items():
+        assert torch.equal(v, ckpt['backbone.' + k]), k
+    back = model.state_dict()
+    assert back.keys() == ckpt.keys()
+    for k, v in ckpt.items():
+        assert torch.equal(back[k], v), k
